@@ -146,7 +146,9 @@ def test_network_oracle_matches_reference_golden(golden_dir, cfg_path):
 
 
 def test_oracle_network_other_resolutions_match_reference_golden(cfg_path, golden_dir):
-    """the oracle network at a multi-resolution training shape and a small one vs the reference's logits (make_golden.py main_multires)"""
+    """the oracle network at a multi-resolution training shape and a small one vs the reference's logits (make_golden.py main_multires).
+    Bit for bit on the CPU that generated the goldens; another CPU's convolution kernels sum in another order (4e-6 of the largest
+    logit measured on a second x86 host), hence 2e-5."""
     import torch
     from oracle.darknet_ref import RefDarknet
     from singleshotpose_b200 import synth
@@ -155,6 +157,8 @@ def test_oracle_network_other_resolutions_match_reference_golden(cfg_path, golde
     m = RefDarknet(cfg_path).train()
     for (h, w, seed) in ((352, 480, 5), (224, 224, 6)):
         with torch.no_grad():
-            o = m(synth.images(1, h, w, seed=seed))
-        assert torch.equal(o, torch.from_numpy(g["logits_%dx%d" % (h, w)]))
+            o = m(synth.images(1, h, w, seed=seed)).numpy()
+        want = g["logits_%dx%d" % (h, w)]
+        assert o.shape == want.shape
+        assert np.abs(o - want).max() / np.abs(want).max() < 2e-5, (h, w)
 
